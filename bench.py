@@ -50,6 +50,9 @@ def parse_args():
                     help="torch.optim.Adam implementation: PyTorch's fused kernel (default) or its foreach form: 98.8 -> 97.6 ms")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-eager", action="store_true", help="skip the reference-eager-on-this-GPU baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, run the timed step once more from the starting weights and write what "
+                         "it computed to DIR/<name>.npy (float32, rank 0; see dump_outputs)")
     return ap.parse_args()
 
 
@@ -338,6 +341,33 @@ def roofline_entry(name, kt, pk, ops, traffic):
             "ms_per_step": kt["ms_per_step"], "peak_source": pk["source"]}
 
 
+DUMP_ROWS = 1024          # rows of h / z kept by --dump-outputs (all of them at the default batch)
+DUMP_PARAM_SAMPLE = 1 << 22
+
+
+def dump_outputs(out_dir, loss, outputs, model):
+    """The results of one training step as DIR/<name>.npy, float32, 25 MiB at most: ``loss``; ``h_i``, ``h_j``,
+    ``z_i``, ``z_j`` (the encoder outputs and embeddings of both views, a seeded sample of DUMP_ROWS rows above that
+    batch); ``grads``: a fixed seeded sample of DUMP_PARAM_SAMPLE of the 18.4 M trainable entries' gradients
+    (concatenated in named_parameters order).  The updated parameters are left out: where a gradient is analytically
+    zero (biases in front of a train-mode BatchNorm) Adam turns its rounding noise into a +-lr step of either sign."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": np.array(loss, dtype=np.float32)}
+    for name, t in zip(("h_i", "h_j", "z_i", "z_j"), outputs):
+        t = t.detach()
+        if t.shape[0] > DUMP_ROWS:
+            rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(1))[:DUMP_ROWS].sort().values
+            t = t[rows.to(t.device)]
+        arrays[name] = t.float().cpu().numpy()
+    params = [p for p in model.parameters() if p.requires_grad]
+    flat_g = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).detach().reshape(-1) for p in params])
+    pick = torch.randperm(flat_g.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_PARAM_SAMPLE].sort().values
+    arrays["grads"] = flat_g[pick.to(flat_g.device)].float().cpu().numpy()
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     from grafp_b200 import _native, ops, synth
     from grafp_b200.encoder.graph_encoder import GraphEncoder
@@ -361,6 +391,7 @@ def run_ours(args):
     cfg["bsz_train"] = args.batch
     torch.manual_seed(0)
     model = SimCLR(cfg, GraphEncoder(cfg=cfg, in_channels=cfg["n_filters"], k=3)).to(dev).train()
+    start = {k: v.clone() for k, v in model.state_dict().items()} if args.dump_outputs else None
     net = model
     # whole step incl. the gradient all-reduce as one CUDA graph per rank (GRAFP_BENCH_DP_GRAPH=0: DistributedDataParallel, eager)
     graph_dp = world > 1 and (args.graph == "on" or (args.graph == "auto" and os.environ.get("GRAFP_BENCH_DP_GRAPH", "1") != "0"))
@@ -386,7 +417,11 @@ def run_ours(args):
     dev_i, dev_j = host_i.to(dev), host_j.to(dev)
     h2d_bytes = host_i.numel() * 4 + host_j.numel() * 4
 
+    last_outputs = []
+
     def loss_of(h_i, h_j, z_i, z_j):
+        if args.dump_outputs:   # under a CUDA graph these are its static outputs, refreshed by every replay
+            last_outputs[:] = [h_i, h_j, z_i, z_j]
         # global-batch negatives like the reference's DataParallel gather (train.py:69-71); the loss runs in fp32
         return global_ntxent_loss(z_i.float(), z_j.float(), cfg)
 
@@ -466,6 +501,21 @@ def run_ours(args):
     e3.record()
     barrier()
     ms_e2e = e2.elapsed_time(e3)
+    if args.dump_outputs:
+        # The state after the warmup and timed steps carries their rounding noise (unordered fp32 reductions, cuDNN's
+        # timed algorithm choice), which Adam and the k-NN's near-ties amplify from step to step; so the dumped step is
+        # the timed one (same graph or eager step, same inputs) run again from the starting weights and a fresh Adam state.
+        with torch.no_grad():
+            for k, v in model.state_dict().items():
+                v.copy_(start[k])
+            for state in opt.state.values():
+                for t in state.values():
+                    if torch.is_tensor(t):
+                        t.zero_()
+        loss = step(host_i, host_j) if use_graph else step(host_i.to(dev), host_j.to(dev))
+        barrier()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, loss.item(), last_outputs, model)
 
     ms_instr = ms_resident
     if use_graph:

@@ -9,6 +9,8 @@ them on seeded synthetic inputs and writes ``*.npz`` files next to this script. 
 fixtures are what pins ``oracle/grafp_oracle.py`` to the reference
 (tests/test_oracle_golden.py) and what the GPU parity tests replay on the B200 box,
 where /root/reference does not exist.
+
+``fingerprints.npz`` is the exception: it comes from the oracle at full size on the GPU (see make_fingerprints).
 """
 import os
 import sys
@@ -368,10 +370,66 @@ def make_retrieval(ref):
     save("retrieval", q_specs=q_specs, pick=pick, db=db, queries=q, top1=top1, margin=margin, **buffers)
 
 
+def make_fingerprints():
+    """configs[4] at its stated size (10 000 DB segments, 1 000 queries, top-1 by inner product) through the reference
+    algorithm as oracle/grafp_oracle.py restates it (pinned to the upstream modules by the fixtures above), run eager in
+    fp32 on a B200 with TF32 off, as test_fingerprint_generation_at_size_matches_the_reference_on_the_same_gpu runs
+    everything else.  Needs the built library and a CUDA device, no upstream checkout:
+
+        python tests/golden/make_golden.py fingerprints
+
+    BatchNorm running statistics as a trained checkpoint would carry them: one train-mode pass (momentum 1) of the
+    device model over 512 DB segments; the test loads the stored statistics, so both sides evaluate the same function.
+    Stored: those statistics, the query hits and their margins over the runner-up, and a seeded sample of 768 DB
+    fingerprints (the whole DB is 5 MB)."""
+    from oracle import grafp_oracle as O
+    from grafp_b200.encoder.graph_encoder import GraphEncoder
+    from grafp_b200.simclr.simclr import SimCLR
+    dev = torch.device("cuda")
+    torch.backends.cudnn.enabled = True
+    torch.backends.cudnn.allow_tf32 = False
+    torch.backends.cuda.matmul.allow_tf32 = False
+    cfg = dict(synth.DEFAULT_CFG)
+    n_db, n_q, chunk = 10_000, 1_000, 128
+    torch.manual_seed(0)
+    model = SimCLR(cfg, GraphEncoder(cfg=cfg, in_channels=cfg["n_filters"], k=3))
+    load_synth(model, 303)
+    db_specs, _ = synth.synth_spec(n_db, 7)
+    model.to(dev).train()
+    for m in model.modules():
+        if isinstance(m, torch.nn.BatchNorm2d):
+            m.momentum = 1.0
+    with torch.no_grad():
+        model(db_specs[:512].to(dev), db_specs[:512].to(dev))
+    p = {k: v.detach().clone() for k, v in model.state_dict().items()}
+    buffers = {f"buf.{k}": v for k, v in p.items() if k.endswith("running_mean") or k.endswith("running_var")}
+    pick = torch.randperm(n_db, generator=torch.Generator().manual_seed(8))[:n_q]
+    q_specs = db_specs[pick] + 0.02 * torch.randn(n_q, 64, 32, generator=torch.Generator().manual_seed(9))
+
+    def fingerprints(specs):
+        with torch.no_grad():
+            return torch.cat([O.simclr_forward(p, specs[lo:lo + chunk].to(dev), specs[:1].to(dev), False, k=3)[2]
+                              for lo in range(0, specs.shape[0], chunk)])
+
+    db, q = fingerprints(db_specs), fingerprints(q_specs)
+    sims = q @ db.T
+    best2 = sims.topk(2, dim=1).values
+    top1 = sims.argmax(1).cpu()
+    sample = torch.randperm(n_db, generator=torch.Generator().manual_seed(10))[:768].sort().values
+    print(torch.cuda.get_device_name(), "fingerprints at size: hits", int((top1 == pick).sum()), f"/ {n_q}")
+    save("fingerprints", top1=top1.int(), margin=best2[:, 0] - best2[:, 1], sample=sample.int(),
+         db_sample=db[sample.to(dev)], **buffers)
+
+
 def main():
+    only = set(sys.argv[1:])
+    if "fingerprints" in only:
+        make_fingerprints()
+        only.discard("fingerprints")
+        if not only:
+            return
     ref = _reference_import.load()
     torch.manual_seed(0)
-    only = set(sys.argv[1:])
     for name, fn in (("knn", make_knn), ("knn_cos", make_knn_cos), ("aggregate", make_aggregate), ("gconv", make_gconv), ("gconv_r2", make_gconv_r2),
                      ("grapher", make_grapher), ("encoder", make_encoder), ("simclr", make_simclr), ("retrieval", make_retrieval)):
         if not only or name in only:
