@@ -12,6 +12,7 @@ import pytest
 import torch
 
 import golden_io as gio
+from golden_io import _default_kernel_options, _exact_fp32_library_math  # noqa: F401  (autouse: TF32 off, default options)
 from grafp_b200 import _native, ops, synth
 from grafp_b200.encoder.gcn_lib import torch_edge, torch_nn, torch_vertex
 from grafp_b200.encoder.graph_encoder import GraphEncoder
@@ -22,30 +23,6 @@ from oracle import grafp_oracle as O
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
 REL_TOL = 1e-4
-
-
-@pytest.fixture(autouse=True)
-def _exact_fp32_library_math():
-    # the parity bar is fp32: keep cuDNN / cuBLAS off TF32 for the PyTorch layers around our kernels
-    old = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
-    torch.backends.cudnn.allow_tf32 = False
-    torch.backends.cuda.matmul.allow_tf32 = False
-    yield
-    torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = old
-
-
-_OPTION_DEFAULTS = {"mr_fwd_form": 2, "mr_bwd_form": 2, "knn_epilogue": 0, "edge_bwd_row": 1, "gather_row": 1, "edge_row": 1,
-                    "maxk_row": 1, "bn_reverse": 1, "bn_persistent": 1, "bn_l2_keep_mb": 80, "check_index": 0, "conv_gemm": 1}
-
-
-@pytest.fixture(autouse=True)
-def _default_kernel_options():
-    """Kernel-selection options are process-wide: every test starts from, and leaves, the defaults."""
-    for name, value in _OPTION_DEFAULTS.items():
-        ops.set_option(name, value)
-    yield
-    for name, value in _OPTION_DEFAULTS.items():
-        ops.set_option(name, value)
 
 
 def load_synth(module, seed):
@@ -969,12 +946,6 @@ def test_ntxent_row_shards_equal_the_full_problem():
                                      1.0 / tau, stream) == -1     # odd bounds would split a pair
 
 
-def _bn_moments(ws, C):
-    """The per-channel (sum, sum of squares) doubles inside a BatchNorm workspace (256-byte aligned, bn_fused.cu)."""
-    off = (-ws.data_ptr()) % 256
-    return ws[off:off + 16 * C].view(torch.float64).view(2, C)
-
-
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
 @pytest.mark.parametrize("shape", [(4, 256, 64, 64), (3, 500, 128, 256), (2, 129, 256, 320), (5, 77, 8, 24), (1, 1024, 2048, 512),
                                    (2, 300, 96, 1024), (1, 2, 64, 128)])
@@ -994,7 +965,7 @@ def test_conv1x1_stats_kernel(shape, dtype):
     ref = torch.nn.functional.conv2d(x.double(), w.double())
     err = gio.rel_err(h.double().cpu(), ref.cpu())
     assert err < (1.5e-3 if dtype == torch.float32 else 4e-3), err
-    m = _bn_moments(ws, Cout).cpu()
+    m = gio.bn_moments(ws, Cout).cpu()
     hd = h.double().permute(0, 2, 3, 1).reshape(B * N, Cout).cpu()
     s1, s2 = hd.sum(0), (hd * hd).sum(0)
     assert float((m[1] - s2).abs().max() / s2.abs().max()) < 3e-6    # fp32 partial sums per 64-row half tile
@@ -1022,7 +993,7 @@ def test_conv1x1_stats_kernel_grouped(shape, dtype):
     ref = torch.nn.functional.conv2d(x.double(), w.double(), groups=G)
     err = gio.rel_err(h.double().cpu(), ref.cpu())
     assert err < (1.5e-3 if dtype == torch.float32 else 4e-3), err
-    m = _bn_moments(ws, Cout).cpu()
+    m = gio.bn_moments(ws, Cout).cpu()
     hd = h.double().permute(0, 2, 3, 1).reshape(B * N, Cout).cpu()
     s1, s2 = hd.sum(0), (hd * hd).sum(0)
     assert float((m[1] - s2).abs().max() / s2.abs().max()) < 3e-6
@@ -1040,7 +1011,7 @@ def test_conv1x1_stats_large_mean():
     x[:, 0] = 1000.0                                   # a constant input channel: a large per-channel offset of y
     w = (torch.randn(Cout, Cin, 1, 1, generator=g) / 8).to(DEV)
     h, ws = ops._conv1x1_stats_call(ops._native.load(), x, w)
-    m = _bn_moments(ws, Cout).cpu()
+    m = gio.bn_moments(ws, Cout).cpu()
     hd = h.double().permute(0, 2, 3, 1).reshape(B * N, Cout).cpu()
     var = m[1] / (B * N) - (m[0] / (B * N)) ** 2
     assert float(hd.mean(0).abs().median() / hd.std(0).max()) > 10.0     # the offset dominates in most channels
