@@ -52,6 +52,9 @@ SIGNATURES = {
     "grafp_conv1x1_bn_stats_supported": (_i, [_c.c_longlong, _i, _i, _i, _i]),
     "grafp_conv1x1_bn_stats_fwd": (_i, [_vp] * 3 + [_c.c_longlong, _i, _i, _i, _i, _vp, _sz, _vp]),
     "grafp_bn_train_fwd_from_moments": (_i, [_vp] * 11 + [_c.c_longlong, _i, _c.c_float, _c.c_float, _i, _i, _vp, _sz, _vp]),
+    "grafp_search_prepare": (_i, [_vp, _c.c_longlong, _i, _vp, _vp, _vp, _vp]),
+    "grafp_search_workspace_bytes": (_sz, [_i] * 4),
+    "grafp_search_fwd": (_i, [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
 }
 
 ABI_VERSION = 7

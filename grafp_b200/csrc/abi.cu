@@ -369,7 +369,56 @@ int grafp_max_over_k_bwd(const void* grad_out, const uint8_t* argmax, void* grad
 
 }  // extern "C"
 
+namespace grafp {
+static int search_envelope(const char* fn, int n_q, int n_db, int d, int k) {
+  GRAFP_REQUIRE(n_q > 0 && n_db > 0 && d > 0 && k > 0, GRAFP_EINVAL, "%s: n_q, n_db, d and k must be positive", fn);
+  GRAFP_REQUIRE(d % 8 == 0 && d >= 64 && d <= 256, GRAFP_EUNSUPPORTED, "%s: d = %d is not a multiple of 8 in [64, 256]", fn, d);
+  GRAFP_REQUIRE(k <= GRAFP_KNN_MAX_K, GRAFP_EUNSUPPORTED, "%s: k = %d exceeds %d", fn, k, GRAFP_KNN_MAX_K);
+  GRAFP_REQUIRE(k <= n_db, GRAFP_EINVAL, "%s: k = %d exceeds the %d database rows", fn, k, n_db);
+  return GRAFP_OK;
+}
+}  // namespace grafp
+
 extern "C" {
+
+int grafp_search_prepare(const float* rows, long long n, int d, void* hi, void* lo, float* sq, void* stream) {
+  clear_error();
+  GRAFP_REQUIRE(n > 0 && d > 0, GRAFP_EINVAL, "grafp_search_prepare: n and d must be positive");
+  GRAFP_REQUIRE(d % 8 == 0 && d >= 64 && d <= 256, GRAFP_EUNSUPPORTED, "grafp_search_prepare: d = %d is not a multiple of 8 in [64, 256]", d);
+  GRAFP_REQUIRE(rows && hi && lo && sq, GRAFP_EINVAL, "grafp_search_prepare: rows, hi, lo and sq must be non-null");
+  { int rc = require_device("grafp_search_prepare"); if (rc != GRAFP_OK) return rc; }
+  { int rc = require_device_ptr("grafp_search_prepare", "rows", rows); if (rc) return rc; }
+  { int rc = require_device_ptr("grafp_search_prepare", "hi", hi); if (rc) return rc; }
+  { int rc = require_device_ptr("grafp_search_prepare", "lo", lo); if (rc) return rc; }
+  { int rc = require_device_ptr("grafp_search_prepare", "sq", sq); if (rc) return rc; }
+  return launch_knn_normalize<float>(rows, static_cast<float*>(hi), static_cast<float*>(lo), sq, n, d, 3, false,
+                                     static_cast<cudaStream_t>(stream));
+}
+
+size_t grafp_search_workspace_bytes(int n_q, int n_db, int d, int k) {
+  if (search_envelope("grafp_search_workspace_bytes", n_q, n_db, d, k) != GRAFP_OK) return 0;
+  return search_workspace_bytes(n_q, n_db, d, k);
+}
+
+int grafp_search_fwd(const float* q, int n_q, const void* hi, const void* lo, const float* sq, int n_db, int d, int k,
+                     int64_t* ids, float* dist, void* workspace, size_t workspace_bytes, void* stream) {
+  clear_error();
+  { int rc = search_envelope("grafp_search_fwd", n_q, n_db, d, k); if (rc != GRAFP_OK) return rc; }
+  GRAFP_REQUIRE(q && hi && lo && sq && ids && dist && workspace, GRAFP_EINVAL,
+                "grafp_search_fwd: q, hi, lo, sq, ids, dist and workspace must be non-null");
+  GRAFP_REQUIRE(aligned16(q) && aligned16(hi) && aligned16(lo) && aligned16(sq), GRAFP_EINVAL,
+                "grafp_search_fwd: q, hi, lo and sq must be 16-byte aligned");
+  { int rc = require_device("grafp_search_fwd"); if (rc != GRAFP_OK) return rc; }
+  { int rc = require_device_ptr("grafp_search_fwd", "q", q); if (rc) return rc; }
+  { int rc = require_device_ptr("grafp_search_fwd", "hi", hi); if (rc) return rc; }
+  { int rc = require_device_ptr("grafp_search_fwd", "lo", lo); if (rc) return rc; }
+  { int rc = require_device_ptr("grafp_search_fwd", "sq", sq); if (rc) return rc; }
+  { int rc = require_device_ptr("grafp_search_fwd", "ids", ids); if (rc) return rc; }
+  { int rc = require_device_ptr("grafp_search_fwd", "dist", dist); if (rc) return rc; }
+  { int rc = require_device_ptr("grafp_search_fwd", "workspace", workspace); if (rc) return rc; }
+  return launch_search(q, n_q, hi, lo, sq, n_db, d, k, reinterpret_cast<long long*>(ids), dist, workspace, workspace_bytes,
+                       static_cast<cudaStream_t>(stream));
+}
 
 size_t grafp_bn_workspace_bytes(int C) { return C > 0 ? bn_workspace_bytes(C) : 0; }
 

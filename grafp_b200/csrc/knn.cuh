@@ -33,4 +33,10 @@ int launch_knn_tc2(const void* xhi, const void* xlo, const float* xsq, const voi
                    const float* ysq, long long* nn_idx, int* nn_idx32, int B, int N, int M, int C, int K, int k_out,
                    int stride, int dtype, bool self, void* bounds, cudaStream_t s);
 
+// exact flat search (knn_tc2.cu): fp16 planes + |x|^2 of n_db database rows (launch_knn_normalize, mode 3, no
+// normalisation), queries fp32 (n_q, d); ids / dist (n_q, k) ascending.  0 bytes: no plan for the shape.
+size_t search_workspace_bytes(int n_q, int n_db, int d, int k);
+int launch_search(const float* q, int n_q, const void* hi, const void* lo, const float* sq, int n_db, int d, int k,
+                  long long* ids, float* dist, void* workspace, size_t workspace_bytes, cudaStream_t s);
+
 }  // namespace grafp

@@ -27,6 +27,8 @@
 
 #include <cuda_fp16.h>
 
+#include <algorithm>
+#include <climits>
 #include <cstdlib>
 #include <cstring>
 
@@ -292,9 +294,11 @@ struct GroupTop {
       for (int g = 0; g < 4; ++g) offer(m[g], (key0 >> 3) + g, &v[8 * g]);
     }
   }
-  // exact ranking of the listed groups' keys into `top` (ascending key order, so ties keep the lower id)
-  template <int KREG, bool YS_SHARED>
-  __device__ __forceinline__ void finish(TopK<KREG>& top, uint32_t ys_addr, const float* ys_glob) {
+  // exact ranking of the listed groups' keys into `top` (ascending key order, so ties keep the lower id).
+  // RAGGED: the key count `nkeys` need not be a multiple of 32; columns past it were masked to -inf before `scan32`
+  // (so their distance is +inf) and their |y|^2 is not read.
+  template <int KREG, bool YS_SHARED, bool RAGGED = false>
+  __device__ __forceinline__ void finish(TopK<KREG>& top, uint32_t ys_addr, const float* ys_glob, int nkeys = 0) {
 #pragma unroll
     for (int i = 0; i < KG - 1; ++i) {  // sort by group id (the slot bits cannot reorder distinct ids)
 #pragma unroll
@@ -314,6 +318,9 @@ struct GroupTop {
       if constexpr (YS_SHARED) {
         asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(y[0]), "=f"(y[1]), "=f"(y[2]), "=f"(y[3]) : "r"(ys_addr + 32u * gid));
         asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(y[4]), "=f"(y[5]), "=f"(y[6]), "=f"(y[7]) : "r"(ys_addr + 32u * gid + 16u));
+      } else if (RAGGED && 8 * gid + 8 > nkeys) {
+#pragma unroll
+        for (int e = 0; e < 8; ++e) y[e] = (8 * gid + e < nkeys) ? __ldg(ys_glob + 8 * gid + e) : 0.f;
       } else {
         const float4 y0 = __ldg(reinterpret_cast<const float4*>(ys_glob + 8 * gid));
         const float4 y1 = __ldg(reinterpret_cast<const float4*>(ys_glob + 8 * gid) + 1);
@@ -334,6 +341,10 @@ __host__ __device__ constexpr uint32_t epi_warp_bytes() {
   return QS > 0 ? (uint32_t)QS * 512u : (QS < 0 ? (uint32_t)KREG * 1024u : 0u);
 }
 constexpr float kUnitNormTol = 1e-4f;  // group-maxima selection needs | |y|^2 - 1 | below this for every key of the segment
+// The flat search also bounds the spread of |y|^2 over the slice: ranking groups by the raw accumulator misorders two keys
+// by at most that spread, and 1e-6 keeps it below the fp32 tie band 4 sqrt(d) 2^-23 (3.8e-6 at d = 64) that exact search
+// is held to.  Normalised fp32 rows spread by a few 1e-7.
+constexpr float kSearchUnitSpread = 1e-6f;
 
 __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
@@ -451,19 +462,29 @@ __device__ __forceinline__ void tmem_dealloc(uint32_t base, uint32_t cols) {
 // ---------------------------------------------------------------------------------------------
 // resident queries, streamed keys
 // ---------------------------------------------------------------------------------------------
-template <int NH, int BN, int KREG, int QS>
+// SPLIT (the flat search, B = 1): blockIdx.y selects the key slice [s0, s0 + slice_len) of the database.  Key ids, the
+// |y|^2 range test and the round bounds (per slice and query) are slice-local, and instead of `emit` the epilogue
+// writes the row's best (distance, slice-local id) pairs of ranks rank0 .. to part[(slice * N + q) * k_out + rank]
+// for the merge kernel.
+template <int NH, int BN, int KREG, int QS, bool SPLIT = false>
 __global__ void __launch_bounds__((4 * NH + 2) * 32, 1)
 knn_stream_kernel(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ CUtensorMap tm_x_lo,
                   const __grid_constant__ CUtensorMap tm_y_hi, const __grid_constant__ CUtensorMap tm_y_lo,
                   const float* __restrict__ xsq, const float* __restrict__ ysq, long long* __restrict__ nn_idx,
                   int* __restrict__ nn_idx32, int N, int M, int C, int k_out, int stride, int stages,
-                  float2* bounds, int rank0, int more_rounds) {
+                  float2* bounds, int rank0, int more_rounds, int slice_len, float2* __restrict__ part) {
   constexpr int kProducerWarp = 4 * NH, kMmaWarp = 4 * NH + 1;
   constexpr uint32_t kTmemCols = 2 * NH * BN;  // two accumulator sets of NH tiles, BN keys wide
   constexpr uint32_t kKeyBlockBytes = 2 * BN * BK * 2;  // hi + lo plane of BN keys x 64 channels
   extern __shared__ unsigned char smem_raw[];
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int num_kc = (C + BK - 1) / BK;
+  int s0 = 0;  // first key of this CTA's slice; M becomes the slice's key count
+  if constexpr (SPLIT) {
+    s0 = blockIdx.y * slice_len;
+    M = min(slice_len, M - s0);
+    ysq += s0;
+  }
   const int num_tiles = (M + BN - 1) / BN;
   unsigned char* q_base = smem;                                    // [NH][num_kc] blocks
   unsigned char* ring = q_base + (size_t)NH * num_kc * kBlockBytes; // [stages] blocks
@@ -478,7 +499,7 @@ knn_stream_kernel(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_cons
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  const int b = blockIdx.y;
+  const int b = SPLIT ? 0 : blockIdx.y;
   const int m0 = blockIdx.x * (BM * NH);
 
   if (threadIdx.x == 0) {
@@ -512,8 +533,8 @@ knn_stream_kernel(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_cons
           const uint32_t full = bar_full + 8 * s;
           mbar_arrive_expect_tx(full, kKeyBlockBytes);
           const uint32_t dst = smem_u32(ring + (size_t)s * kKeyBlockBytes);
-          tma_load_3d(dst, &tm_y_hi, full, c * BK, t * BN, b);
-          tma_load_3d(dst + kKeyBlockBytes / 2, &tm_y_lo, full, c * BK, t * BN, b);
+          tma_load_3d(dst, &tm_y_hi, full, c * BK, s0 + t * BN, b);
+          tma_load_3d(dst + kKeyBlockBytes / 2, &tm_y_lo, full, c * BK, s0 + t * BN, b);
           if (++s == stages) { s = 0; ph ^= 1; }
         }
       }
@@ -550,12 +571,19 @@ knn_stream_kernel(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_cons
     const int quarter = warp & 3;
     const int r = quarter * 32 + lane;
     const int q = m0 + h * BM + r;
-    const float sq_i = (q < N) ? xsq[(long long)b * N + q] : 0.f;
+    // SPLIT: n_q need not fill the query block.  A padding row (TMA zero fill: acc = 0) with |x|^2 = 0 would have a
+    // negative threshold once its list is full and take every key as a candidate, pacing its warp and, through the
+    // TMEM release, the CTA; |x|^2 = +inf makes its threshold NaN, so it never has one.
+    const float sq_i = (q < N) ? xsq[(long long)b * N + q] : (SPLIT ? INFINITY : 0.f);
     const float* ysq_b = ysq + (long long)b * M;
     const bool ys_vec = (M & 3) == 0 && (reinterpret_cast<uintptr_t>(ysq) & 15) == 0;
     TopK<KREG> top;
     top.init(sq_i);
-    if (q < N) load_bound<KREG>(top, bounds, (long long)b * N + q, rank0);
+    if constexpr (SPLIT) {
+      if (q < N) load_bound<KREG>(top, bounds, (long long)blockIdx.y * N + q, rank0);  // round bounds per (slice, query)
+    } else {
+      if (q < N) load_bound<KREG>(top, bounds, (long long)b * N + q, rank0);
+    }
     if constexpr (QS > 0) top.queue_init(smem_u32(queue) + (uint32_t)warp * (QS * 512), lane, QS);
     GroupTop<(QS < 0) ? KREG : 1> gt;
     if constexpr (QS < 0) gt.init(smem_u32(queue) + (uint32_t)warp * epi_warp_bytes<QS, KREG>(), lane);
@@ -571,6 +599,7 @@ knn_stream_kernel(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_cons
       }
       top.set_tile(mn);
       unit_keys = mn >= 1.f - kUnitNormTol && mx <= 1.f + kUnitNormTol;  // warp- and CTA-uniform (same keys for all)
+      if constexpr (SPLIT) unit_keys = unit_keys && mx - mn <= kSearchUnitSpread;
     }
     for (int t = 0; t < num_tiles; ++t) {
       const int as = t & 1;
@@ -589,6 +618,12 @@ knn_stream_kernel(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_cons
             uint32_t v[32];
             tmem_ld32(trow + c0, v);
             tmem_ld_wait();
+            if constexpr (SPLIT) {  // the ragged last slice: TMA zero-filled columns (acc = 0) must not rank as groups
+              if (c0 + 32 > ncols) {
+#pragma unroll
+                for (int j = 0; j < 32; ++j) v[j] = (c0 + j < ncols) ? v[j] : 0xff800000u;
+              }
+            }
             gt.scan32(v, t * BN + c0);
           }
         } else {
@@ -606,11 +641,20 @@ knn_stream_kernel(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_cons
       if (lane == 0) mbar_arrive(bar_tempty + 8 * as);
     }
     if constexpr (QS < 0) {
-      if (unit_keys) gt.template finish<KREG, false>(top, 0u, ysq_b);
+      if (unit_keys) gt.template finish<KREG, false, SPLIT>(top, 0u, ysq_b, M);
     }
     if (q < N) {
-      emit<KREG>(top, nn_idx, nn_idx32, ((long long)b * N + q) * k_out, k_out, stride, rank0);
-      store_bound<KREG>(top, bounds, (long long)b * N + q, more_rounds);
+      if constexpr (SPLIT) {
+        const long long row = (long long)blockIdx.y * N + q;
+        float2* out = part + row * k_out;
+#pragma unroll
+        for (int p = 0; p < KREG; ++p)
+          if (rank0 + p < k_out) out[rank0 + p] = make_float2(top.d[p], __int_as_float(top.id[p]));
+        store_bound<KREG>(top, bounds, row, more_rounds);
+      } else {
+        emit<KREG>(top, nn_idx, nn_idx32, ((long long)b * N + q) * k_out, k_out, stride, rank0);
+        store_bound<KREG>(top, bounds, (long long)b * N + q, more_rounds);
+      }
     }
   }
 
@@ -837,19 +881,26 @@ struct Round {
   int rank0, more;
 };
 
-template <int NH, int BN, int KREG, int QS>
+// key slices of the flat search (SPLIT kernels): `count` slices of `len` keys, the last one ragged
+struct Slices {
+  int count = 0, len = 0;
+  float2* part = nullptr;
+};
+
+template <int NH, int BN, int KREG, int QS, bool SPLIT>
 static int launch_stream(const CUtensorMap& xh, const CUtensorMap& xl, const CUtensorMap& yh, const CUtensorMap& yl,
                          const float* xsq, const float* ysq, long long* nn_idx, int* nn_idx32, int B, int N, int M, int C,
-                         int k_out, int stride, int stages, Round r, cudaStream_t s) {
+                         int k_out, int stride, int stages, Round r, Slices sl, cudaStream_t s) {
   static DeviceOnce once;
-  if (int rc = set_smem(knn_stream_kernel<NH, BN, KREG, QS>, &once, "knn_stream")) return rc;
+  if (int rc = set_smem(knn_stream_kernel<NH, BN, KREG, QS, SPLIT>, &once, "knn_stream")) return rc;
   const int num_kc = (C + BK - 1) / BK;
   const size_t smem = (size_t)(NH * num_kc) * kBlockBytes + (size_t)stages * (2 * BN * BK * 2) +
                       (size_t)(4 * NH) * epi_warp_bytes<QS, KREG>() + kMiscBytes;
-  dim3 grid((N + BM * NH - 1) / (BM * NH), B);
-  knn_stream_kernel<NH, BN, KREG, QS><<<grid, (4 * NH + 2) * 32, smem, s>>>(xh, xl, yh, yl, xsq, ysq, nn_idx, nn_idx32, N, M,
-                                                                       C, k_out, stride, stages, r.bounds, r.rank0, r.more);
-  return check_launch("knn_stream");
+  // query blocks along x (the fastest launch index): the CTAs that share a key slice run in the same wave
+  dim3 grid((N + BM * NH - 1) / (BM * NH), SPLIT ? sl.count : B);
+  knn_stream_kernel<NH, BN, KREG, QS, SPLIT><<<grid, (4 * NH + 2) * 32, smem, s>>>(
+      xh, xl, yh, yl, xsq, ysq, nn_idx, nn_idx32, N, M, C, k_out, stride, stages, r.bounds, r.rank0, r.more, sl.len, sl.part);
+  return check_launch(SPLIT ? "knn_search" : "knn_stream");
 }
 
 template <int NH, int KREG, int QS>
@@ -871,20 +922,11 @@ struct Plan {
   int kind = 0, nh = 0, bn = 0, stages = 0, qs = 0;
 };
 
-static Plan plan_with(int N, int M, int C, int K, int dtype, bool self, bool allow_group_max);
+static Plan plan_with(int N, int C, bool self, int qs);
 
 static Plan plan(int N, int M, int C, int K, int dtype, bool self) {
-  // the group-maxima selection needs 3 KB of spill slots per epilogue warp next to the resident queries; where that does
-  // not fit (wide separate key sets) the vote-gated form of the same kernels is used
-  Plan p = plan_with(N, M, C, K, dtype, self, true);
-  if (p.kind == 0) p = plan_with(N, M, C, K, dtype, self, false);
-  return p;
-}
-
-static Plan plan_with(int N, int M, int C, int K, int dtype, bool self, bool allow_group_max) {
-  Plan p;
   // (dtype: the planes are fp16 whatever the input was - the normalise kernel reads fp32 or bf16 rows)
-  if ((dtype != GRAFP_F32 && dtype != GRAFP_BF16) || C % 8 != 0 || C < BK || N < BM || M < BM || K < 1 || K > GRAFP_KNN_MAX_K) return p;
+  if ((dtype != GRAFP_F32 && dtype != GRAFP_BF16) || C % 8 != 0 || C < BK || N < BM || M < BM || K < 1 || K > GRAFP_KNN_MAX_K) return Plan{};
   // Which selection epilogue.  K > 8 (16-entry lists, rounds) exists in the candidate-queue form only.  For K <= 8 both
   // exist and neither dominates: on features with independent rows (random point clouds: scripts/bench_ops.py, the
   // configs[3] stress) the queue form is faster (stage 0: 385 vs 429 us) because some lane of a warp has a candidate
@@ -895,9 +937,20 @@ static Plan plan_with(int N, int M, int C, int K, int dtype, bool self, bool all
   // K <= 3 with a key count that is a multiple of 32 (every encoder stage): the group-maxima selection (qs = -1).
   const int epi = option(OPT_KNN_EPILOGUE);
   const bool force_queue = epi == 2;
-  const bool group_max = allow_group_max && K <= 3 && M % 32 == 0 && (epi == 3 || (epi == 0 && kGroupMaxDefault));
+  const bool group_max = K <= 3 && M % 32 == 0 && (epi == 3 || (epi == 0 && kGroupMaxDefault));
+  const int qs = (K <= 8 && !force_queue) ? 0 : kQueueSlots;
+  // the group-maxima selection needs 3 KB of spill slots per epilogue warp next to the resident queries; where that does
+  // not fit (wide separate key sets) the vote-gated form of the same kernels is used
+  Plan p = plan_with(N, C, self, group_max ? -1 : qs);
+  if (p.kind == 0 && group_max) p = plan_with(N, C, self, qs);
+  return p;
+}
+
+// kernel, query block, key tile and ring depth for N queries of C channels with the selection form qs
+static Plan plan_with(int N, int C, bool self, int qs) {
+  Plan p;
   const bool no_nh4 = false, bn128 = false;
-  p.qs = group_max ? -1 : ((K <= 8 && !force_queue) ? 0 : kQueueSlots);
+  p.qs = qs;
   const int num_kc = (C + BK - 1) / BK;
   const uint32_t budget = kSmemLimit - kMiscBytes;
   auto queue_bytes = [&](int nh) { return (uint32_t)(4 * nh) * (p.qs > 0 ? (uint32_t)p.qs * 512u : (p.qs < 0 ? 3u * 1024u : 0u)); };
@@ -951,15 +1004,18 @@ struct Args {
   int* nn_idx32;
   int B, N, M, C, k_out, stride;
   cudaStream_t s;
+  Slices sl;
 };
 
-template <int KR, int QS>
+template <int KR, int QS, bool SPLIT = false>
 static int launch_planned(const Plan& p, const Args& a, Round r) {
 #define GRAFP_SELF(NH_) launch_self<NH_, KR, QS>(*a.xh, *a.xl, a.xsq, a.nn_idx, a.nn_idx32, a.B, a.N, a.C, a.k_out, a.stride, p.stages, r, a.s)
 #define GRAFP_STREAM(NH_, BN_)                                                                                          \
-  launch_stream<NH_, BN_, KR, QS>(*a.xh, *a.xl, *a.yh, *a.yl, a.xsq, a.ysq, a.nn_idx, a.nn_idx32, a.B, a.N, a.M, a.C, a.k_out, \
-                                  a.stride, p.stages, r, a.s)
-  if (p.kind == 1) return p.nh == 1 ? GRAFP_SELF(1) : GRAFP_SELF(2);
+  launch_stream<NH_, BN_, KR, QS, SPLIT>(*a.xh, *a.xl, *a.yh, *a.yl, a.xsq, a.ysq, a.nn_idx, a.nn_idx32, a.B, a.N, a.M, a.C, \
+                                         a.k_out, a.stride, p.stages, r, a.sl, a.s)
+  if constexpr (!SPLIT) {
+    if (p.kind == 1) return p.nh == 1 ? GRAFP_SELF(1) : GRAFP_SELF(2);
+  }
   if (p.nh == 4) return GRAFP_STREAM(4, 64);
   if (p.bn == 64) return p.nh == 2 ? GRAFP_STREAM(2, 64) : GRAFP_STREAM(1, 64);
   return p.nh == 2 ? GRAFP_STREAM(2, 128) : GRAFP_STREAM(1, 128);
@@ -985,7 +1041,7 @@ int launch_knn_tc2(const void* xhi, const void* xlo, const float* xsq, const voi
     set_error("knn_tc2: cuTensorMapEncodeTiled failed (driver entry point unavailable or bad shape)");
     return GRAFP_EUNSUPPORTED;
   }
-  const Args a = {&xh, &xl, &yh, &yl, xsq, ysq, nn_idx, nn_idx32, B, N, M, C, k_out, stride, s};
+  const Args a = {&xh, &xl, &yh, &yl, xsq, ysq, nn_idx, nn_idx32, B, N, M, C, k_out, stride, s, Slices{}};
   const Round one = {nullptr, 0, 0};
   if (K <= 3) {
     if (p.qs < 0) return launch_planned<3, -1>(p, a, one);
@@ -1004,6 +1060,152 @@ int launch_knn_tc2(const void* xhi, const void* xlo, const float* xsq, const voi
     if (int rc = launch_planned<16, kQueueSlots>(p, a, rd)) return rc;
   }
   return GRAFP_OK;
+}
+
+}  // namespace grafp
+
+// ---------------------------------------------------------------------------------------------
+// exact flat search: the key-sliced stream kernel + a merge of the per-slice lists
+// ---------------------------------------------------------------------------------------------
+namespace grafp {
+namespace tc2 {
+
+constexpr int kMaxSlices = 1024;          // merge cursors per query (one byte each, k <= 128)
+constexpr int kMaxSliceLen = 1 << 26;     // group ids (slice-local key / 8) stay below GroupTop::kInvalid
+constexpr int kMergeWarps = 4;
+
+struct SearchPlan {
+  Plan p;
+  int slices = 0, slice_len = 0;
+};
+
+// Selection form from k alone.  Database rows are independent, the case where K1 measured the candidate queue ahead of
+// the vote-gated scan; k <= 3 takes the group maxima, on slices whose keys are unit-norm (the vote-gated scan elsewhere).
+// Slices: (query blocks x slices) >= 2 CTAs per SM, each slice a whole number of key tiles (64 or 128 keys, so also of
+// the 32-key chunks of the group maxima) and at least two of them.
+static SearchPlan search_plan(int n_q, int n_db, int d, int k) {
+  SearchPlan sp;
+  sp.p = plan_with(n_q, d, false, k <= 3 ? -1 : kQueueSlots);
+  if (sp.p.kind != 2) return SearchPlan{};
+  const long long qblocks = (n_q + BM * sp.p.nh - 1) / (BM * sp.p.nh);
+  const long long want = (2LL * num_sms() + qblocks - 1) / qblocks;
+  const long long tile = sp.p.bn;
+  long long len = ((long long)n_db + want - 1) / want;
+  len = (len + tile - 1) / tile * tile;
+  len = std::max(len, 2 * tile);
+  len = std::min(len, (long long)kMaxSliceLen);
+  sp.slice_len = (int)len;
+  sp.slices = (int)(((long long)n_db + len - 1) / len);
+  if (sp.slices > kMaxSlices) return SearchPlan{};
+  return sp;
+}
+
+struct SearchLayout {
+  size_t plane, qsq, bounds, part, total;
+};
+static size_t align1k(size_t v) { return (v + 1023) / 1024 * 1024; }
+static SearchLayout search_layout(int n_q, int d, int k, int slices) {
+  SearchLayout l;
+  l.plane = align1k((size_t)n_q * d * 2);                              // query hi / lo planes (fp16)
+  l.qsq = align1k((size_t)n_q * 4);                                    // |q|^2
+  l.bounds = k > 16 ? align1k((size_t)slices * n_q * 8) : 0;           // round hand-over per (slice, query)
+  l.part = align1k((size_t)slices * n_q * k * 8);                      // per-slice lists (dist, slice-local id)
+  l.total = 2 * l.plane + l.qsq + l.bounds + l.part + 1024;            // + base alignment
+  return l;
+}
+
+// One warp per query: k steps of a lexicographic (dist, global id) minimum over the heads of the slices' sorted lists.
+// Slices are disjoint ascending id ranges and each list is exact, so the result is the single-pass top-k bit for bit
+// (for the group maxima: up to keys closer than the slice's |y|^2 spread, see kSearchUnitSpread).
+__global__ void __launch_bounds__(kMergeWarps * 32)
+search_merge_kernel(const float2* __restrict__ part, int slices, int slice_len, int N, int k, long long* __restrict__ ids,
+                    float* __restrict__ dist) {
+  __shared__ unsigned char cursor[kMergeWarps][kMaxSlices];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int q = blockIdx.x * kMergeWarps + warp;
+  if (q >= N) return;  // warp-uniform; the warps share no data
+  unsigned char* cur = cursor[warp];
+  for (int s = lane; s < slices; s += 32) cur[s] = 0;
+  __syncwarp();
+  float bd;
+  int bid, bs;
+  auto rescan = [&]() {  // this lane's best head over its slices lane, lane + 32, ...
+    bd = INFINITY; bid = INT_MAX; bs = -1;
+    for (int s = lane; s < slices; s += 32) {
+      if (cur[s] >= k) continue;
+      const float2 v = part[((long long)s * N + q) * k + cur[s]];
+      const int gid = s * slice_len + __float_as_int(v.y);
+      if (bs < 0 || v.x < bd || (v.x == bd && gid < bid)) { bd = v.x; bid = gid; bs = s; }
+    }
+  };
+  rescan();
+  for (int r = 0; r < k; ++r) {
+    float md = bd;
+    int mid = bid;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float od = __shfl_xor_sync(0xffffffffu, md, o);
+      const int oid = __shfl_xor_sync(0xffffffffu, mid, o);
+      if (od < md || (od == md && oid < mid)) { md = od; mid = oid; }
+    }
+    if (lane == 0) { ids[(long long)q * k + r] = mid; dist[(long long)q * k + r] = md; }
+    if (bs >= 0 && bid == mid && bd == md) {  // the one lane holding the winner advances that slice
+      ++cur[bs];
+      rescan();
+    }
+    __syncwarp();
+  }
+}
+
+}  // namespace tc2
+
+size_t search_workspace_bytes(int n_q, int n_db, int d, int k) {
+  using namespace tc2;
+  const SearchPlan sp = search_plan(n_q, n_db, d, k);
+  return sp.p.kind == 2 ? search_layout(n_q, d, k, sp.slices).total : 0;
+}
+
+int launch_search(const float* q, int n_q, const void* hi, const void* lo, const float* sq, int n_db, int d, int k,
+                  long long* ids, float* dist, void* workspace, size_t workspace_bytes, cudaStream_t s) {
+  using namespace tc2;
+  const SearchPlan sp = search_plan(n_q, n_db, d, k);
+  if (sp.p.kind != 2) {
+    set_error("grafp_search_fwd: no kernel plan for n_q=%d n_db=%d d=%d k=%d", n_q, n_db, d, k);
+    return GRAFP_EUNSUPPORTED;
+  }
+  const SearchLayout l = search_layout(n_q, d, k, sp.slices);
+  if (workspace_bytes < l.total) {
+    set_error("grafp_search_fwd: workspace of %zu bytes is smaller than grafp_search_workspace_bytes() = %zu", workspace_bytes, l.total);
+    return GRAFP_EWORKSPACE;
+  }
+  char* base = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~uintptr_t(1023));
+  float* q_hi = reinterpret_cast<float*>(base);
+  float* q_lo = reinterpret_cast<float*>(base + l.plane);
+  float* q_sq = reinterpret_cast<float*>(base + 2 * l.plane);
+  float2* bounds = l.bounds ? reinterpret_cast<float2*>(base + 2 * l.plane + l.qsq) : nullptr;
+  float2* part = reinterpret_cast<float2*>(base + 2 * l.plane + l.qsq + l.bounds);
+  if (int rc = launch_knn_normalize<float>(q, q_hi, q_lo, q_sq, n_q, d, 3, false, s)) return rc;
+  CUtensorMap xh, xl, yh, yl;
+  if (!make_map_f16(&xh, q_hi, 1, n_q, d) || !make_map_f16(&xl, q_lo, 1, n_q, d) || !make_map_f16(&yh, hi, 1, n_db, d, sp.p.bn) ||
+      !make_map_f16(&yl, lo, 1, n_db, d, sp.p.bn)) {
+    set_error("grafp_search_fwd: cuTensorMapEncodeTiled failed (driver entry point unavailable or bad shape)");
+    return GRAFP_EUNSUPPORTED;
+  }
+  const Args a = {&xh, &xl, &yh, &yl, q_sq, sq, nullptr, nullptr, 1, n_q, n_db, d, k, 1, s, Slices{sp.slices, sp.slice_len, part}};
+  const Round one = {nullptr, 0, 0};
+  int rc = GRAFP_OK;
+  if (k <= 3) {
+    rc = launch_planned<3, -1, true>(sp.p, a, one);
+  } else if (k <= 8) {
+    rc = launch_planned<8, kQueueSlots, true>(sp.p, a, one);
+  } else {
+    const int rounds = (k + 15) / 16;
+    for (int r = 0; r < rounds && rc == GRAFP_OK; ++r) rc = launch_planned<16, kQueueSlots, true>(sp.p, a, {bounds, 16 * r, r + 1 < rounds ? 1 : 0});
+  }
+  if (rc != GRAFP_OK) return rc;
+  search_merge_kernel<<<(n_q + kMergeWarps - 1) / kMergeWarps, kMergeWarps * 32, 0, s>>>(part, sp.slices, sp.slice_len, n_q, k,
+                                                                                     ids, dist);
+  return check_launch("search_merge");
 }
 
 }  // namespace grafp

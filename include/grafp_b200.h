@@ -307,6 +307,26 @@ int grafp_peak_extract_fwd(const float* spec, const float* weight, const float* 
 int grafp_peak_extract_bwd(const float* spec, const float* out, const float* grad_out, void* partial, size_t partial_bytes,
                            float* dweight, float* dbias, int B, int H, int W, int F, int kh, int kw, int stride_h, void* stream);
 
+/*
+ * Exact flat search: the k nearest database rows of every query in squared L2 distance (faiss IndexFlatL2.search).
+ *   grafp_search_prepare: fp16 planes hi / lo (n, d) of rows * 2^12 and sq (n) = |row|^2 (fp32) for the caller's rows
+ *     (n, d) float32; called on appended rows through pointer offsets, so a database is prepared once.
+ *   grafp_search_fwd: q (n_q, d) float32 against the n_db prepared rows; ids (n_q, k) int64 and dist (n_q, k) float32,
+ *     ascending by (dist, id) - equal distances keep the lower id.  dist = (|q|^2 + (-2 q.x)) + |x|^2 in fp32.
+ *     The database is cut into key slices searched in parallel and their lists merged; the result does not depend on
+ *     the slicing or on the other queries of the batch - for k <= 3 on unit-norm rows up to near-ties: keys whose
+ *     distances differ by less than the spread of the rows' |x|^2 (<= 1e-6) may be ordered or picked either way.
+ *   Precondition: every database and query row has L2 norm <= 1 + 1e-4 (the fp16 plane split and the selection
+ *   thresholds assume it; unit-norm fingerprints satisfy it).  Not checked here.
+ *   Envelope: d % 8 == 0 and 64 <= d <= 256, 1 <= k <= 128, k <= n_db, n_q >= 1 (else GRAFP_EUNSUPPORTED / GRAFP_EINVAL).
+ *   workspace: grafp_search_workspace_bytes(n_q, n_db, d, k) bytes (0 outside the envelope).  Nothing is allocated and
+ *   nothing synchronises; the kernels run on `stream` of the current device.
+ */
+int grafp_search_prepare(const float* rows, long long n, int d, void* hi, void* lo, float* sq, void* stream);
+size_t grafp_search_workspace_bytes(int n_q, int n_db, int d, int k);
+int grafp_search_fwd(const float* q, int n_q, const void* hi, const void* lo, const float* sq, int n_db, int d, int k,
+                     int64_t* ids, float* dist, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
